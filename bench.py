@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — audio-seconds generated per wall-second on the Tango hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 One "step" = one pass of the hot path over one batch of synthetic prompts: `denoise_steps` (200) CFG denoising steps
@@ -17,6 +17,9 @@ Printed JSON (rank 0, one line):
   cpu_baseline  the oracle port timed on this box's host cores on a bounded sample (N=1 only)
 `--impl reference` times the reference's CPU arithmetic (oracle port; the Python reference itself cannot travel to the
 GPU box) on the same config / metric.
+`--dump-outputs DIR` writes what the last timed step returned on rank 0 (latents, float and int16 waveforms) as
+DIR/<name>.npy in float32. Inputs, weights and noise are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 from __future__ import annotations
 
@@ -244,6 +247,7 @@ def run_ours(args):
     gen = torch.Generator(device=dev).manual_seed(1234 + rank)
 
     decode_ms = []
+    last = {}   # the latest pass's outputs: persistent device buffers, overwritten by the next pass
 
     def one_pass_device():
         lat = t.model.inference(prompts, t.scheduler, args.denoise_steps, args.guidance, prompt_embeds=embeds_d,
@@ -255,6 +259,7 @@ def run_ours(args):
         out = t.vae.decode_rows_to_waveform(rows, B_, H, W)
         d1.record()
         decode_ms.append((d0, d1))
+        last.update(latents=lat, waveform=out[0], waveform_int16=out[1])
         return out
 
     def one_pass_e2e():
@@ -289,6 +294,8 @@ def run_ours(args):
     barrier()
     dev_ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:   # before the legs below reuse the buffers
+        dump_outputs(args.dump_outputs, last)
     launches = (L.launch_count() - n0) + graph_launches
     dec_ms = float(np.mean([a.elapsed_time(b) for a, b in decode_ms[-args.steps:]]))
     dev_ms = parallel.max_over_ranks(dev_ms, dev)
@@ -551,6 +558,25 @@ def cpu_baseline(args):
     return {"value": v, "unit": "audio-s/s", "cores": ref.cores, "kind": "port", "sample": ref.describe(t_step, 1, t_dec, 2)}
 
 
+DUMP_LIMIT = 64 * 10**6   # bytes over all files written by --dump-outputs, .npy headers included
+
+
+def dump_outputs(path, tensors):
+    """Each tensor as path/<name>.npy in float32 (the int16 waveform converts exactly). The default workload writes
+    ~11.5 MB; beyond DUMP_LIMIT every array is replaced by the same seeded random sample of its flattened elements, in
+    proportion to its size, so that runs with the same arguments still compare element for element."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in tensors.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    budget = DUMP_LIMIT - 1024 * len(arrays)
+    for name, a in arrays.items():
+        if total > budget:
+            k = a.size * budget // total
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, k, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+    print(f"bench.py: wrote {', '.join(sorted(arrays))} to {path}", file=sys.stderr, flush=True)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -571,7 +597,13 @@ def main():
                     help="--impl reference: stop timing further steps once this much wall time has been used")
     ap.add_argument("--no-parity-mode", action="store_true", help="skip the split-precision (1e-3 mode) leg")
     ap.add_argument("--no-extra-configs", action="store_true", help="at --gpus 8: skip the c4 / c5 legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step (rank 0) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     knobs = sorted(k for k in os.environ if k.startswith("TNG_"))
     if knobs:
         raise SystemExit(f"bench.py: refusing to run with experiment knobs set in the environment: {knobs}")

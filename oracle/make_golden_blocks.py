@@ -3,8 +3,8 @@
 mustango/diffusers/tests/test_layers_utils.py builds each block with `torch.manual_seed(0)` default initialisation
 and compares an output slice with hard-coded constants. The constants live in tests/test_oracle_pins.py (cited there);
 this script reproduces the seeded inputs + module weights through the UNMODIFIED reference modules, checks that the
-reference still meets its constants on this torch build, and stores inputs + weights so the oracle's block functions can
-be checked against the same constants anywhere.
+reference still meets its constants on this torch build, and stores inputs + weights (tests/golden/block_known_answers/,
+one file per block) so the oracle's block functions can be checked against the same constants anywhere.
 
     python -m oracle.make_golden_blocks
 """
@@ -114,8 +114,15 @@ def main():
         out.update({f"{name}." + k: v for k, v in blk.state_dict().items()})
         out[f"{name}_x_sum"] = inp["hidden_states"].double().sum().float()
 
-    np.savez_compressed(os.path.join(GOLD, "block_known_answers.npz"), **{k: v.numpy() for k, v in out.items()})
-    print("wrote", os.path.join(GOLD, "block_known_answers.npz"), f"({len(out)} arrays)")
+    # one file per block (keys keep the block's prefix), so that no fixture file grows past 1 MB
+    blocks = sorted(EXPECTED) + sorted(UNET_BLOCKS)
+    os.makedirs(os.path.join(GOLD, "block_known_answers"), exist_ok=True)
+    for name in blocks:
+        part = {k: v.numpy() for k, v in out.items() if k.startswith((name + ".", name + "_"))}
+        path = os.path.join(GOLD, "block_known_answers", name + ".npz")
+        np.savez_compressed(path, **part)
+        print("wrote", path, f"({len(part)} arrays)")
+    assert sum(k.startswith((n + ".", n + "_")) for k in out for n in blocks) == len(out)
 
 
 if __name__ == "__main__":

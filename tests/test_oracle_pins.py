@@ -197,7 +197,7 @@ def test_tiny_stft_frontend_golden():
 # Known-answer slices hard-coded in the diffusers fork's own block tests (mustango/diffusers/tests/test_layers_utils.py):
 # ResnetBlock2D default :226-240, Upsample2D with conv :131-141, Downsample2D with conv / padding 1 :200-210,
 # Transformer2DModel with cross attention :394-418. Each test seeds torch with 0, draws the input, then builds the module
-# with default initialisation; oracle/make_golden_blocks.py stores those module weights (tests/golden/block_known_answers.npz).
+# with default initialisation; oracle/make_golden_blocks.py stores those module weights (tests/golden/block_known_answers/).
 BLOCK_KNOWN = {
     "resnet": [-1.9010, -0.2974, -0.8245, -1.3533, 0.8742, -0.9645, -2.0584, 1.3387, -0.4746],
     "upsample": [0.7145, 1.3773, 0.3492, 0.8448, 1.0839, -0.3341, 0.5956, 0.1250, -0.4841],
@@ -216,7 +216,7 @@ def _seeded_input(gd, name, shape):
 
 @pytest.mark.parametrize("name", sorted(BLOCK_KNOWN))
 def test_oracle_blocks_meet_reference_known_answers(name):
-    gd = gold("block_known_answers.npz")
+    gd = gold(f"block_known_answers/{name}.npz")
     sd = {k[len(name) + 1:]: torch.from_numpy(gd[k]) for k in gd.files if k.startswith(name + ".")}
     if name == "resnet":
         x = _seeded_input(gd, name, (1, 32, 64, 64))
@@ -252,7 +252,7 @@ UNET_BLOCK_KNOWN = {
 
 @pytest.mark.parametrize("name", sorted(UNET_BLOCK_KNOWN))
 def test_oracle_unet_blocks_meet_reference_known_answers(name):
-    gd = gold("block_known_answers.npz")
+    gd = gold(f"block_known_answers/{name}.npz")
     sd = {k[len(name) + 1:]: torch.from_numpy(gd[k]) for k in gd.files if k.startswith(name + ".")}
     # the harness builds the attention blocks with 1x1-conv projections; same arithmetic as the linear form
     sd = {k: (v[:, :, 0, 0] if k.endswith(("proj_in.weight", "proj_out.weight")) and v.dim() == 4 else v)
