@@ -223,17 +223,11 @@ class View:
         return View(t, ld if C_ is None else C_, W, H, NB, ld, W * ld, H * W * ld)
 
 
-def conv_gemm(views: Sequence[View], groups: Sequence[tuple], weight: torch.Tensor, W: int, H: int, NB: int, *,
-              bias=None, rowvec=None, res=None, alpha: float = 1.0, accumulate: bool = False, out_f32=None,
-              out_bf16=None, act: int = ACT_NONE, act_param: float = 0.0, split_off: int = 0, block_n: int = 0,
-              ld_f32: Optional[int] = None, ld_bf16: Optional[int] = None, ldr: Optional[int] = None,
-              rowvec_ld: int = 0, algo_k: Optional[int] = None, gn_stats: Optional[torch.Tensor] = None,
-              stats_hw: int = 0) -> None:
-    """Launch tng_conv_gemm. groups: (view, a_c0, dw, dh, b_k0, nkb). weight: bf16 [Ncols, Ktot].
-    algo_k: algorithmic reduction length (taps * Cin of the reference op) for the profiler's FLOP count.
-    gn_stats: fp64 [images, Ncols, 2] per-channel GroupNorm accumulators of the fp32 output (zeroed by the caller),
-    images of stats_hw rows each."""
-    lib = load()
+def _gemm_desc(views: Sequence[View], groups: Sequence[tuple], weight: torch.Tensor, W: int, H: int, NB: int, *,
+               bias=None, rowvec=None, res=None, alpha: float = 1.0, accumulate: bool = False, out_f32=None,
+               out_bf16=None, act: int = ACT_NONE, act_param: float = 0.0, split_off: int = 0, block_n: int = 0,
+               ld_f32: Optional[int] = None, ld_bf16: Optional[int] = None, ldr: Optional[int] = None,
+               rowvec_ld: int = 0, gn_stats: Optional[torch.Tensor] = None, stats_hw: int = 0) -> GemmDesc:
     d = GemmDesc()
     require_cuda(weight, bias, rowvec, res, out_f32, out_bf16)
     assert weight.dtype == torch.bfloat16 and weight.stride(1) == 1
@@ -271,13 +265,39 @@ def conv_gemm(views: Sequence[View], groups: Sequence[tuple], weight: torch.Tens
         require_cuda(gn_stats)
         assert gn_stats.dtype == torch.float64 and gn_stats.is_contiguous() and stats_hw > 0
         d.gn_stats, d.stats_hw = gn_stats.data_ptr(), stats_hw
+    return d
+
+
+def _plan(d: GemmDesc) -> tuple:
+    bn, mode, ks = C.c_int32(0), C.c_int32(0), C.c_int32(0)
+    check(load().tng_gemm_plan(C.byref(d), C.byref(bn), C.byref(mode), C.byref(ks)), "tng_gemm_plan")
+    return bn.value, mode.value, ks.value
+
+
+def gemm_plan(views: Sequence[View], groups: Sequence[tuple], weight: torch.Tensor, W: int, H: int, NB: int,
+              **kw) -> tuple:
+    """(block_n, mode, ksplit) that tng_conv_gemm would launch for these arguments (same signature as conv_gemm):
+    the N tile, 1 = one CTA per SM / 4 = CTA pair on a 256 x 2*block_n tile, and the split-K factor."""
+    kw.pop("algo_k", None)
+    return _plan(_gemm_desc(views, groups, weight, W, H, NB, **kw))
+
+
+def conv_gemm(views: Sequence[View], groups: Sequence[tuple], weight: torch.Tensor, W: int, H: int, NB: int, *,
+              algo_k: Optional[int] = None, **kw) -> None:
+    """Launch tng_conv_gemm. groups: (view, a_c0, dw, dh, b_k0, nkb). weight: bf16 [Ncols, Ktot].
+    Epilogue keywords: bias, rowvec (+ rowvec_ld), res (+ ldr), alpha, accumulate, out_f32 (+ ld_f32), out_bf16
+    (+ ld_bf16), act, act_param, split_off, block_n, gn_stats, stats_hw.
+    algo_k: algorithmic reduction length (taps * Cin of the reference op) for the profiler's FLOP count.
+    gn_stats: fp64 [images, Ncols, 2] per-channel GroupNorm accumulators of the fp32 output (zeroed by the caller),
+    images of stats_hw rows each."""
+    lib = load()
+    d = _gemm_desc(views, groups, weight, W, H, NB, **kw)
     if PROF.enabled:
         k_alg = algo_k if algo_k is not None else sum(g[5] for g in groups) * 64
         flops = 2.0 * W * H * NB * weight.shape[0] * k_alg
-        bn, mode, ks = C.c_int32(0), C.c_int32(0), C.c_int32(0)
-        check(lib.tng_gemm_plan(C.byref(d), C.byref(bn), C.byref(mode), C.byref(ks)), "tng_gemm_plan")
-        tag = {1: "1cta", 2: "mcast", 3: "pair", 4: "pair2"}.get(mode.value, str(mode.value))
-        fam = f"gemm_tc<{bn.value},{tag}" + (",splitk>" if ks.value > 1 else ">")
+        bn, mode, ks = _plan(d)
+        tag = {1: "1cta", 2: "mcast", 3: "pair", 4: "pair2"}.get(mode, str(mode))
+        fam = f"gemm_tc<{bn},{tag}" + (",splitk>" if ks > 1 else ">")
         PROF.timed(fam, flops, 0, lambda: check(lib.tng_conv_gemm(C.byref(d), stream_ptr()), "tng_conv_gemm"))
         return
     check(lib.tng_conv_gemm(C.byref(d), stream_ptr()), "tng_conv_gemm")

@@ -21,6 +21,24 @@ def rel_err(a, b):
     return ((a.float() - b.float()).norm() / b.float().norm().clamp_min(1e-12)).item()
 
 
+def run_conv_planned(monkeypatch, *args, **kw):
+    """ops.run_conv, returning ((block_n, mode, ksplit), launches) of the one tng_conv_gemm call it makes: the plan
+    lib.gemm_plan reports for that descriptor, and 1 launch (statistics in the epilogue) or 2 (pass after the GEMM)."""
+    real, seen = L.conv_gemm, []
+
+    def rec(views, groups, weight, W, H, NB, **k):
+        plan = L.gemm_plan(views, groups, weight, W, H, NB, **k)
+        n0 = L.launch_count()
+        real(views, groups, weight, W, H, NB, **k)
+        seen.append((plan, L.launch_count() - n0))
+
+    with monkeypatch.context() as m:
+        m.setattr(L, "conv_gemm", rec)
+        ops.run_conv(*args, **kw)
+    assert len(seen) == 1
+    return seen[0]
+
+
 def nhwc_rows(x):  # [N,C,H,W] -> [N*H*W, C]
     return x.permute(0, 2, 3, 1).reshape(-1, x.shape[1]).contiguous()
 
@@ -68,11 +86,12 @@ def test_conv3x3(cuda, NB, H, W, Cin, Cout):
     assert rel_err(of, ref) < 2e-5
 
 
-@pytest.mark.parametrize("NB,H,W,Cin,Cout,split", [(5, 32, 64, 128, 320, False),     # 40 pair tiles x 1 N pair
-                                                   (20, 16, 16, 128, 640, False),    # 20 x 2, W < 128 pixel tiles
-                                                   (20, 8, 64, 64, 256, True),       # N tile 128 x 2, hi/lo K groups
+# Pair mode needs >= 36 K blocks of 64 (9 taps x Cin / 64, x 3 in split mode) and (pairs) x (N pairs) x 2 >= SMs / 2
+@pytest.mark.parametrize("NB,H,W,Cin,Cout,split", [(5, 32, 64, 256, 320, False),     # 40 pair tiles x 1 N pair
+                                                   (20, 16, 16, 256, 640, False),    # 20 x 2, W < 128 pixel tiles
+                                                   (20, 8, 64, 128, 256, True),      # N tile 128 x 2, hi/lo K groups
                                                    (4, 64, 16, 320, 1280, False)])   # 16 x 4, the UNet level-2 shape
-def test_conv3x3_pair_tiles_two_accumulators(cuda, NB, H, W, Cin, Cout, split):
+def test_conv3x3_pair_tiles_two_accumulators(cuda, monkeypatch, NB, H, W, Cin, Cout, split):
     """Launches large enough for the CTA-pair mode (tcgen05 cta_group::2, 256 x 2*BN output tile per pair, two
     accumulators in a 3-slot TMEM ring): full epilogue with bias, time-embedding row vector, residual, fp32 + bf16
     (SiLU) outputs and the GroupNorm statistics, against torch."""
@@ -88,8 +107,10 @@ def test_conv3x3_pair_tiles_two_accumulators(cuda, NB, H, W, Cin, Cout, split):
     of = torch.full((NB * H * W, Cout), float("nan"), device=cuda)
     ob = torch.zeros(NB * H * W, Cout * (2 if split else 1), device=cuda, dtype=torch.bfloat16)
     st = torch.zeros(NB, Cout, 2, device=cuda, dtype=torch.float64)
-    ops.run_conv(pc, xin, NB, H, W, rowvec=temb, res=res, out_f32=of, out_bf16=ob, act=L.ACT_SILU, gn_stats=st,
-                 stats_hw=H * W)
+    plan, launches = run_conv_planned(monkeypatch, pc, xin, NB, H, W, rowvec=temb, res=res, out_f32=of, out_bf16=ob,
+                                      act=L.ACT_SILU, gn_stats=st, stats_hw=H * W)
+    assert plan == ((128, 4, 1) if split else (160, 4, 1)), f"{plan}: choose a shape that reaches the pair mode again"
+    assert launches == 1      # statistics from the epilogue
     if split:
         ref = F.conv2d(x.double(), w.double(), b.double(), padding=1).float()
     else:
@@ -315,14 +336,17 @@ def test_groupnorm(cuda, C0, C1, act, eps):
     assert rel_err(raw[:, :Cc].float() + raw[:, Cc:].float(), xc) < 1e-5
 
 
-@pytest.mark.parametrize("shape", [(16, 8, 4, 128, 320, 1, "full tiles: epilogue"),     # NB, H, W, Cin, Cout, taps
-                                   (4, 16, 16, 64, 640, 9, "3x3 conv, full tiles: epilogue"),
-                                   (3, 4, 8, 64, 64, 9, "partial tiles: pass after the GEMM"),
-                                   (2, 2, 32, 1280, 1280, 9, "under-filled split-K launch: pass after the GEMM")])
-def test_conv_gemm_emits_groupnorm_statistics(cuda, shape):
+# NB, H, W, Cin, Cout, taps, (plan, launches) with an fp32 output and with a bf16-only output; plan = (block_n, mode,
+# ksplit), launches 1 = statistics from the epilogue, 2 = pass after the GEMM
+@pytest.mark.parametrize("shape", [(16, 8, 4, 128, 320, 1, ((160, 1, 1), 1), ((160, 1, 1), 1)),     # full tiles
+                                   (4, 16, 16, 64, 640, 9, ((128, 1, 1), 1), ((128, 1, 1), 1)),     # 3x3, full tiles
+                                   (3, 4, 8, 64, 64, 9, ((64, 1, 1), 2), ((64, 1, 1), 2)),          # partial tiles
+                                   # under-filled: split-K with the fp32 output, full N tiles of 128 with bf16 only
+                                   (2, 2, 32, 1280, 1280, 9, ((160, 1, 2), 2), ((128, 1, 1), 1))])
+def test_conv_gemm_emits_groupnorm_statistics(cuda, monkeypatch, shape):
     """tng_conv_gemm(gn_stats=...): per-(image, channel) sum / sum of squares of the fp32 output, accumulated from the
     epilogue (or by the follow-up pass when tiles are partial / split-K), must equal the column sums of what was stored."""
-    NB, H, W, Cin, Cout, taps, _ = shape
+    NB, H, W, Cin, Cout, taps, plan_f32, plan_bf16 = shape
     g = torch.Generator(device="cpu").manual_seed(Cout + taps)
     k = 3 if taps == 9 else 1
     w = torch.randn(Cout, Cin, k, k, generator=g) * (Cin * taps) ** -0.5
@@ -332,7 +356,9 @@ def test_conv_gemm_emits_groupnorm_statistics(cuda, shape):
     pc = PackedConv(w if k == 3 else w[:, :, 0, 0], b, split=False, device=cuda)
     out = torch.zeros(NB * H * W, Cout, device=cuda)
     st = torch.zeros(NB, Cout, 2, device=cuda, dtype=torch.float64)
-    run_conv(pc, bf(x).to(cuda), NB, H, W, res=res if taps == 1 else None, out_f32=out, gn_stats=st, stats_hw=H * W)
+    got = run_conv_planned(monkeypatch, pc, bf(x).to(cuda), NB, H, W, res=res if taps == 1 else None, out_f32=out,
+                           gn_stats=st, stats_hw=H * W)
+    assert got == plan_f32
     torch.cuda.synchronize()
     o = out.double().view(NB, H * W, Cout)
     assert rel_err(st[..., 0], o.sum(1)) < 1e-6 and rel_err(st[..., 1], (o * o).sum(1)) < 1e-6
@@ -345,7 +371,9 @@ def test_conv_gemm_emits_groupnorm_statistics(cuda, shape):
     # rounding of the fp32 sums
     ob = torch.zeros(NB * H * W, Cout, device=cuda, dtype=torch.bfloat16)
     st2 = torch.zeros(NB, Cout, 2, device=cuda, dtype=torch.float64)
-    run_conv(pc, bf(x).to(cuda), NB, H, W, res=res if taps == 1 else None, out_bf16=ob, gn_stats=st2, stats_hw=H * W)
+    got = run_conv_planned(monkeypatch, pc, bf(x).to(cuda), NB, H, W, res=res if taps == 1 else None, out_bf16=ob,
+                           gn_stats=st2, stats_hw=H * W)
+    assert got == plan_bf16
     torch.cuda.synchronize()
     assert rel_err(ob, out) < 5e-3
     assert rel_err(st2[..., 1], (o * o).sum(1)) < 5e-3 and rel_err(st2[..., 0], o.sum(1)) < 2e-2
@@ -522,7 +550,7 @@ def test_gated_tanh_gelu_epilogue(cuda):
 
 
 @pytest.mark.parametrize("NB,H,W,Cin,Cout,sc", [(16, 32, 2, 1280, 1280, 0), (5, 32, 2, 640, 320, 0), (16, 32, 2, 1280, 1280, 640)])
-def test_conv3x3_underfilled_split_k(cuda, NB, H, W, Cin, Cout, sc):
+def test_conv3x3_underfilled_split_k(cuda, monkeypatch, NB, H, W, Cin, Cout, sc):
     """Under-filled launches with a long reduction (the 32x2 level of the UNet) take the split-K path: two CTAs per
     output tile red.add their fp32 partials into a zeroed output; bias / time vector / residual enter once; a fused
     1x1 shortcut rides along as an extra k-group. The 5-image case has a ragged last M tile."""
@@ -538,15 +566,16 @@ def test_conv3x3_underfilled_split_k(cuda, NB, H, W, Cin, Cout, sc):
         ws = (torch.randn(Cout, sc, 1, 1, generator=g) / math.sqrt(sc)).to(cuda)
         bs = torch.randn(Cout, generator=g).to(cuda)
         pc = ops.PackedConv(w, b, split=False, device=cuda, sc_w=ws, sc_b=bs)
-        ops.run_conv(pc, xb, NB, H, W, sc_x=bf(nhwc_rows(xs)), rowvec=temb, out_f32=of)
+        plan, _ = run_conv_planned(monkeypatch, pc, xb, NB, H, W, sc_x=bf(nhwc_rows(xs)), rowvec=temb, out_f32=of)
         ref = F.conv2d(bf(x).float(), bf(w).float(), b, padding=1) + temb[:, :, None, None]
         ref = nhwc_rows(ref + F.conv2d(bf(xs).float(), bf(ws).float(), bs))
     else:
         res = torch.randn(NB * H * W, Cout, generator=g).to(cuda)
         pc = ops.PackedConv(w, b, split=False, device=cuda)
-        ops.run_conv(pc, xb, NB, H, W, rowvec=temb, res=res, alpha=0.5, out_f32=of)
+        plan, _ = run_conv_planned(monkeypatch, pc, xb, NB, H, W, rowvec=temb, res=res, alpha=0.5, out_f32=of)
         ref = F.conv2d(bf(x).float(), bf(w).float(), b, padding=1) + temb[:, :, None, None]
         ref = (nhwc_rows(ref) + res) * 0.5
+    assert plan == (160, 1, 2)
     torch.cuda.synchronize()
     assert rel_err(of, ref) < 2e-5
     of2 = torch.full_like(of, float("nan"))
