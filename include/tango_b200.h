@@ -225,6 +225,29 @@ int tng_sched_step(const float* model_out, int64_t ld_mo, int32_t cfg, float gui
                    int32_t split_off, int64_t B, int64_t C, int64_t HW, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
+ * Fused classifier-free guidance + multistep DPM-Solver / DPM-Solver++ update (one HBM pass).
+ * Replaces: models.py:244-249 and DPMSolverMultistepScheduler.step (scheduling_dpmsolver_multistep.py:
+ *           convert_model_output + the first / second / third order updates).
+ * coef = float[11] {c_s, c_m, c_div, k_s, k0, k1, k2, a1, a2, a3, a4}: fp32 scalars computed on the host with the
+ *        reference's fp32 op order (device pointer). The reference's subtractions are folded into negative
+ *        coefficients (exact in IEEE arithmetic). Every operation below is rounded on its own (no fma contraction):
+ *   v  = u + guidance * (t - u)      (cfg; else v = model_out)
+ *   m0 = (c_s * sample + c_m * v) / c_div                              -> written to m0 (this step's history entry)
+ *   order 1: prev = k_s * sample + k0 * m0
+ *   order 2: D1 = a1 * (m0 - m1);  prev = (k_s * sample + k0 * m0) + k1 * D1
+ *   order 3: E0 = a1 * (m0 - m1);  E1 = a2 * (m1 - m2);  D1 = E0 + a3 * (E0 - E1);  D2 = a4 * (E0 - E1)
+ *            prev = ((k_s * sample + k0 * m0) + k1 * D1) + k2 * D2
+ * model_out: fp32 channels-last [(2)B, HW, ld_mo] (uncond half first when cfg); sample, m1, m2 (the converted outputs
+ * of the previous two steps; read only when `order` needs them), m0, prev: fp32 NCHW [B, C, HW]; prev may alias
+ * sample, m0 may not alias sample, m1 or m2. prev and next_in are optional (at least one). next_in: the channels-last
+ * bf16 UNet input of the next step, exactly as tng_sched_step writes it.
+ */
+int tng_sched_multistep(const float* model_out, int64_t ld_mo, int32_t cfg, float guidance, const float* sample,
+                        const float* m1, const float* m2, const float* coef, int32_t order, float* m0, float* prev,
+                        void* next_in, int64_t ld_in, int32_t split_off, int64_t B, int64_t C, int64_t HW,
+                        void* stream);
+
+/* ---------------------------------------------------------------------------------------------------------
  * Small exact-fp32 pieces.
  * tng_timestep_embedding: get_timestep_embedding (embeddings.py:22-62), flip_sin_to_cos / freq_shift configurable.
  * tng_linear_f32: y = act(x) @ W^T + b for tiny M (TimestepEmbedding, resnet time_emb_proj; embeddings.py:200-212,

@@ -43,7 +43,8 @@ def parse_args(argv: Optional[Sequence[str]] = None) -> argparse.Namespace:
     p.add_argument("--output_root", type=str, default="outputs")
     p.add_argument("--exp_id", type=str, default=None, help="Run id (default: unix time; pass one under torchrun)")
     p.add_argument("--precision", default="bf16", choices=["bf16", "split"])
-    p.add_argument("--scheduler", default="ddpm", choices=["ddpm", "ddim"], help="inference_hf.py uses DDPM")
+    p.add_argument("--scheduler", default="ddpm", choices=["ddpm", "ddim", "dpmsolver++"],
+                   help="inference_hf.py uses DDPM; dpmsolver++ = DPM-Solver++ 2M, meant for 10-25 --num_steps")
     p.add_argument("--latent_h", type=int, default=256, help="latent frames: 256 = 10.24 s (reference)")
     p.add_argument("--seed", type=int, default=None, help="torch.manual_seed for reproducible noise")
     return p.parse_args(argv)
@@ -86,6 +87,9 @@ def build_tango(checkpoint: str, device: str, precision: str, scheduler: str):
     if scheduler == "ddim":
         from .schedulers import DDIMScheduler
         t.scheduler = DDIMScheduler.from_pretrained(t.scheduler_name, subfolder="scheduler")   # same scheduler_config.json
+    elif scheduler == "dpmsolver++":
+        from .schedulers import DPMSolverMultistepScheduler
+        t.scheduler = DPMSolverMultistepScheduler.from_config(t.scheduler.config)   # same betas / prediction type
     return t
 
 

@@ -534,6 +534,65 @@ __global__ void __launch_bounds__(256) sched_step_kernel(const float* mo, long l
   }
 }
 
+// CFG + multistep DPM-Solver(++) update. coef = {c_s, c_m, c_div, k_s, k0, k1, k2, a1, a2, a3, a4} (see
+// include/tango_b200.h); m1 / m2 are read only when `order` needs them. Every product and sum is a separate
+// round-to-nearest operation in the association order of scheduling_dpmsolver_multistep.py, so the result equals the
+// fp32 CPU update bit for bit.
+__global__ void __launch_bounds__(256) sched_multistep_kernel(const float* mo, long long ld_mo, int cfg, float guidance,
+                                                               const float* sample, const float* m1, const float* m2,
+                                                               const float* coef, int order, float* m0_out, float* prev,
+                                                               __nv_bfloat16* next_in, long long ld_in, int split_off,
+                                                               long long B, int C, long long HW) {
+  const float c_s = coef[0], c_m = coef[1], c_div = coef[2], k_s = coef[3], k0 = coef[4], k1 = coef[5], k2 = coef[6];
+  const float a1 = coef[7], a2 = coef[8], a3 = coef[9], a4 = coef[10];
+  const long long total = B * HW * C;
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const int c = static_cast<int>(i % C);
+    const long long hw = (i / C) % HW;
+    const long long b = i / (C * HW);
+    const long long nchw = (b * C + c) * HW + hw;
+    const float s = sample[nchw];
+    float v;
+    if (cfg) {
+      const float u = mo[(b * HW + hw) * ld_mo + c];
+      const float t = mo[((B + b) * HW + hw) * ld_mo + c];
+      v = __fadd_rn(u, __fmul_rn(guidance, __fsub_rn(t, u)));
+    } else {
+      v = mo[(b * HW + hw) * ld_mo + c];
+    }
+    // convert_model_output: x0 (dpmsolver++) or eps (dpmsolver) for every prediction type
+    const float m0 = __fdiv_rn(__fadd_rn(__fmul_rn(c_s, s), __fmul_rn(c_m, v)), c_div);
+    float out = __fadd_rn(__fmul_rn(k_s, s), __fmul_rn(k0, m0));
+    if (order == 2) {
+      const float d1 = __fmul_rn(a1, __fsub_rn(m0, m1[nchw]));
+      out = __fadd_rn(out, __fmul_rn(k1, d1));
+    } else if (order == 3) {
+      const float h1 = m1[nchw];
+      const float e0 = __fmul_rn(a1, __fsub_rn(m0, h1));
+      const float e1 = __fmul_rn(a2, __fsub_rn(h1, m2[nchw]));
+      const float de = __fsub_rn(e0, e1);
+      const float d1 = __fadd_rn(e0, __fmul_rn(a3, de));
+      const float d2 = __fmul_rn(a4, de);
+      out = __fadd_rn(__fadd_rn(out, __fmul_rn(k1, d1)), __fmul_rn(k2, d2));
+    }
+    m0_out[nchw] = m0;
+    if (prev) prev[nchw] = out;
+    if (next_in) {
+      const __nv_bfloat16 hi = __float2bfloat16_rn(out);
+      const __nv_bfloat16 lo = __float2bfloat16_rn(out - __bfloat162float(hi));
+      const long long r0 = (b * HW + hw) * ld_in + c;
+      next_in[r0] = hi;
+      if (split_off > 0) next_in[r0 + split_off] = lo;
+      if (cfg) {
+        const long long r1 = ((B + b) * HW + hw) * ld_in + c;
+        next_in[r1] = hi;
+        if (split_off > 0) next_in[r1 + split_off] = lo;
+      }
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------------------------ time embedding
 __global__ void timestep_embedding_kernel(const float* t, long long n, int dim, int flip, float freq_shift, float* out) {
   const int half = dim / 2;
@@ -863,6 +922,27 @@ extern "C" int tng_sched_step(const float* model_out, int64_t ld_mo, int32_t cfg
                                                                   split_off, B, (int)C, HW);
   count_launch();
   return check_launch("sched_step");
+}
+
+extern "C" int tng_sched_multistep(const float* model_out, int64_t ld_mo, int32_t cfg, float guidance,
+                                   const float* sample, const float* m1, const float* m2, const float* coef,
+                                   int32_t order, float* m0, float* prev, void* next_in, int64_t ld_in,
+                                   int32_t split_off, int64_t B, int64_t C, int64_t HW, void* stream) {
+  if (!model_out || !sample || !coef || !m0 || (!prev && !next_in))
+    return set_error(TNG_EINVAL, "sched_multistep: null argument");
+  if (order < 1 || order > 3) return set_error(TNG_EINVAL, "sched_multistep: order %d not in {1, 2, 3}", (int)order);
+  if ((order >= 2 && !m1) || (order == 3 && !m2))
+    return set_error(TNG_EINVAL, "sched_multistep: order %d needs %s", (int)order, order == 2 ? "m1" : "m1 and m2");
+  if (B <= 0 || C <= 0 || HW <= 0 || ld_mo < C || split_off < 0 || (next_in && ld_in < C + split_off))
+    return set_error(TNG_EINVAL, "sched_multistep: bad shape (B=%lld C=%lld HW=%lld ld_mo=%lld ld_in=%lld split_off=%d)",
+                     (long long)B, (long long)C, (long long)HW, (long long)ld_mo, (long long)ld_in, (int)split_off);
+  if (m0 == m1 || m0 == m2 || m0 == sample || (order == 3 && m1 == m2))
+    return set_error(TNG_EINVAL, "sched_multistep: m0 / m1 / m2 / sample must be distinct buffers");
+  sched_multistep_kernel<<<grid_for(B * C * HW), 256, 0, ST(stream)>>>(
+      model_out, ld_mo, cfg, guidance, sample, m1, m2, coef, order, m0, prev, reinterpret_cast<__nv_bfloat16*>(next_in),
+      ld_in, split_off, B, (int)C, HW);
+  count_launch();
+  return check_launch("sched_multistep");
 }
 
 extern "C" int tng_timestep_embedding(const float* t, int64_t n, int32_t dim, int32_t flip_sin_to_cos, float freq_shift,

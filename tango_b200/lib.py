@@ -24,7 +24,7 @@ SYMBOLS = [
     "tng_groupnorm_stats", "tng_groupnorm_apply", "tng_layernorm", "tng_cast_act", "tng_softmax_rows",
     "tng_transpose_bf16", "tng_sched_step", "tng_timestep_embedding", "tng_linear_f32", "tng_convt_gather",
     "tng_tanh_to_i16", "tng_rmsnorm", "tng_gather_rows", "tng_rel_attention", "tng_stft_frames", "tng_stft_magnitude",
-    "tng_log_clamp", "tng_attention_wide", "tng_gemm_plan",
+    "tng_log_clamp", "tng_attention_wide", "tng_gemm_plan", "tng_sched_multistep",
 ]
 
 
@@ -104,6 +104,7 @@ def load(build_if_missing: bool = True) -> C.CDLL:
         "tng_softmax_rows": [vp, i64, i64, i64, f32, vp, i64, i32, vp],
         "tng_transpose_bf16": [vp, i64, i64, i64, i64, vp, i64, vp],
         "tng_sched_step": [vp, i64, i32, f32, vp, vp, vp, vp, vp, i64, i32, i64, i64, i64, vp],
+        "tng_sched_multistep": [vp, i64, i32, f32, vp, vp, vp, vp, i32, vp, vp, vp, i64, i32, i64, i64, i64, vp],
         "tng_timestep_embedding": [vp, i64, i32, i32, f32, vp, vp],
         "tng_linear_f32": [vp, i64, i64, vp, vp, i64, i32, i32, vp, vp],
         "tng_convt_gather": [vp, i64, i64, i32, i64, i32, i32, i64, vp, vp, vp],
@@ -412,6 +413,21 @@ def sched_step(model_out, cfg, guidance, sample, noise, coef, prev, next_in, *, 
     _call("sched_step", nbytes, load().tng_sched_step, ptr(model_out), 0 if model_out is None else model_out.stride(0),
           int(cfg), guidance, sample.data_ptr(), ptr(noise), coef.data_ptr(), ptr(prev), ptr(next_in),
           0 if next_in is None else next_in.stride(0), split_off, B, Cc, HW, stream_ptr())
+
+
+def sched_multistep(model_out, cfg, guidance, sample, m1, m2, coef, order, m0, prev, next_in, *, B, Cc, HW,
+                    split_off=0):
+    """CFG combine + one multistep DPM-Solver update (coefficient row `coef`, see schedulers.py) + packing of the next
+    UNet input. m1 / m2: the converted model outputs of the previous steps (read for order >= 2 / 3); m0 receives
+    this step's."""
+    require_cuda(model_out, sample, m1, m2, coef, m0, prev, next_in)
+    n = B * Cc * HW
+    reads = (2 if cfg else 1) + 1 + (order >= 2) + (order >= 3)
+    nbytes = n * 4 * (reads + 1 + (prev is not None)) \
+        + (0 if next_in is None else n * (2 if cfg else 1) * (4 if split_off else 2))
+    _call("sched_multistep", nbytes, load().tng_sched_multistep, model_out.data_ptr(), model_out.stride(0), int(cfg),
+          guidance, sample.data_ptr(), ptr(m1), ptr(m2), coef.data_ptr(), int(order), m0.data_ptr(), ptr(prev),
+          ptr(next_in), 0 if next_in is None else next_in.stride(0), split_off, B, Cc, HW, stream_ptr())
 
 
 def timestep_embedding(t, dim, flip_sin_to_cos, freq_shift, out):

@@ -6,8 +6,9 @@ same names, argument meaning, defaults and return types. What changes underneath
 
   * the whole UNet forward is one CUDA-graph replay of hand-written sm_100a kernels (tango_b200/unet.py);
   * cross-attention K/V and the time-embedding projections are computed once per call, not once per step;
-  * CFG combine + scheduler update + re-packing of the next UNet input are ONE kernel (tng_sched_step) fed from a
-    per-step coefficient table, so there is no host sync inside the loop (the reference has two per step);
+  * CFG combine + scheduler update + re-packing of the next UNet input are ONE kernel (tng_sched_step, or
+    tng_sched_multistep for DPMSolverMultistepScheduler) fed from a per-step coefficient table and launched by the
+    scheduler's `fused_step`, so there is no host sync inside the loop (the reference has two per step);
   * a prompt batch can be sharded over the GPUs of one box (tango_b200/parallel.py) — samples are independent.
 
 Text encoding (SURVEY.md §8(f).1): the FLAN-T5 encoder runs on the same kernels (tango_b200/t5.py) whenever its
@@ -33,7 +34,7 @@ import torch
 from . import lib as L
 from . import parallel
 from . import synth
-from .schedulers import DDIMScheduler, DDPMScheduler
+from .schedulers import DDIMScheduler, DDPMScheduler, DPMSolverMultistepScheduler
 from .stft import TacotronSTFT
 from .t5 import T5EncoderModel
 from .unet import UNet2DConditionModel
@@ -352,7 +353,6 @@ class AudioDiffusion:
         if self._temb_cache.get("key") != tkey:   # batch- and data-independent: reuse across calls with the same grid
             self._temb_cache = {"key": tkey, "table": unet.time_embedding_table(timesteps)}
         temb_table = self._temb_cache["table"]                      # [steps, temb_total]
-        coef = sch.coefficient_table(device)                          # [steps, 10]
         s = unet.s
         HW = H * W
         # cfg_on is part of the key: the captured forward bakes in cfg_shared (the CFG shared prefix); so are the device
@@ -413,8 +413,8 @@ class AudioDiffusion:
                     noise = noises[i].to(device, torch.float32).contiguous()
                 else:
                     noise = self.randn_rows((batch_size, Cl, H, W), generator, device, torch.float32, noise_rows)
-            L.sched_step(model_out, cfg_on, float(guidance_scale), sample, noise, coef[i], sample, x_in, B=batch_size,
-                         Cc=Cl, HW=HW, split_off=so)
+            sch.fused_step(i, model_out, cfg_on, float(guidance_scale), sample, noise, x_in, B=batch_size, Cc=Cl, HW=HW,
+                           split_off=so)
             if trace is not None:
                 trace.append(sample.clone())
         ev1.record()
@@ -477,6 +477,8 @@ class Tango:
         self.vae.load_state_dict(synth.synth_state_dict(synth.vae_decoder_param_shapes(), seed))
         if scheduler == "ddim":
             self.scheduler = DDIMScheduler.from_pretrained(None)
+        elif scheduler == "dpmsolver++":   # DPM-Solver++ 2M (midpoint) with the SD-2.1 betas / v_prediction
+            self.scheduler = DPMSolverMultistepScheduler.from_pretrained(None)
         if t5_config is not None:
             if t5_config["d_model"] != ucfg["cross_attention_dim"]:
                 raise ValueError("t5_config['d_model'] must equal the UNet's cross_attention_dim")
